@@ -17,6 +17,10 @@ reports "parity_check": {"n": 128, "mismatches": 0} — at every N.
 
 --impl reference: times the CPU restatement of the reference path (oracle/, kind "port": the Rust reference
 cannot be built here) on the host cores for the same metric / config.
+
+Every timed loop runs --warmup untimed and exactly --steps timed steps.  --dump-outputs DIR writes what each timed
+device path returned in its last timed step (top-10 doc ids, scores and counts) as DIR/<name>.npy; all inputs are
+seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -32,6 +36,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark leaves the source tree as it found it
 
 import numpy as np  # noqa: E402
 import torch  # noqa: E402
@@ -60,6 +65,8 @@ def parse():
     p.add_argument("--cpu-seconds", type=float, default=12.0, help="budget of each cpu_baseline sample")
     p.add_argument("--vector-kernel", default="both", choices=["both", "all", "ffma", "tc", "tc64", "tcb", "tcb64", "tcb256", "filt", "filt256", "filt256p"],
                    help="FP32 FFMA2 scan, tcgen05 scans, or both = ffma + tcb + tcb256 (headline = the fastest: what AUTO picks)")
+    p.add_argument("--dump-outputs", metavar="DIR", default=None,
+                   help="write the results of the last timed step of every device path as DIR/<name>.npy (--impl b200)")
     return p.parse_args()
 
 
@@ -221,6 +228,48 @@ def timed_steps(fn, steps, warmup, world, sampler=None):
     return ms
 
 
+# --dump-outputs: name -> array of what a timed path returned in its last timed step (rank 0; None = not dumping)
+_OUTPUTS = None
+DUMP_BYTES = 60 << 20       # row-sampled above this, so that the .npy files stay under 64 MB in all
+
+
+def keep_keys(name, keys_dev, n, counts_dev=None):
+    """Record the top-10 that a device-resident search left as packed keys (u64 = ordered(score) << 32 | 0xFFFFFFFF - doc_id,
+    0 = empty slot; include/seekstorm_b200.h) as doc ids (float64, -1 = empty) and scores (float32, 0 = empty)."""
+    if _OUTPUTS is None:
+        return
+    k = keys_dev[:n, :TOPK].cpu().numpy().view(np.uint64)
+    o = (k >> np.uint64(32)).astype(np.uint32)
+    bits = np.where(o & np.uint32(0x80000000), o & np.uint32(0x7FFFFFFF), ~o).astype(np.uint32)
+    doc = np.uint32(0xFFFFFFFF) - (k & np.uint64(0xFFFFFFFF)).astype(np.uint32)
+    _OUTPUTS[name + "_ids"] = np.where(k == 0, -1.0, doc.astype(np.float64))
+    _OUTPUTS[name + "_scores"] = np.where(k == 0, np.float32(0), bits.view(np.float32))
+    if counts_dev is not None:
+        _OUTPUTS[name + "_counts"] = counts_dev[:n].cpu().numpy().astype(np.float64)
+
+
+def keep_hits(name, hits, n_hits):
+    """Record host hits (ssb_hit [nq * 10], n_hits [nq]) as doc ids (float64, -1 = empty) and scores (float32, 0 = empty)."""
+    if _OUTPUTS is None:
+        return
+    h = hits[:len(n_hits) * TOPK].reshape(len(n_hits), TOPK)
+    full = np.arange(TOPK)[None, :] < n_hits[:, None]
+    _OUTPUTS[name + "_ids"] = np.where(full, h["doc_id"].astype(np.float64), -1.0)
+    _OUTPUTS[name + "_scores"] = np.where(full, h["score"], np.float32(0))
+
+
+def write_outputs(path):
+    """DIR/<name>.npy for every recorded array.  Above DUMP_BYTES in all, every array keeps the same fraction of its rows (queries),
+    chosen by a fixed seed, so that the files of two runs still line up."""
+    os.makedirs(path, exist_ok=True)
+    total = sum(v.nbytes for v in _OUTPUTS.values())
+    frac = DUMP_BYTES / total if total > DUMP_BYTES else 1.0
+    for name, v in _OUTPUTS.items():
+        if frac < 1.0:
+            v = v[np.sort(np.random.default_rng(0).choice(len(v), max(1, int(len(v) * frac)), replace=False))]
+        np.save(os.path.join(path, name + ".npy"), v)
+
+
 # ----------------------------------------------------------------------------------------------------------------
 def vector_levels(rows, rank, world):
     from seekstorm_b200.parallel import level_range
@@ -274,6 +323,7 @@ def measure_vector_kernel(a, ix, kname, q_host, q_dev, keys, local_rows, rank, w
     step_dev(); torch.cuda.synchronize()
     sampler = ClockSampler(dev.index) if want_clocks else None
     ms = timed_steps(step_dev, a.steps, a.warmup, world, sampler)
+    keep_keys(f"vector_{kname}", keys, a.batch)
     clocks = sampler.stop() if sampler else None
     kern_ns = []
     for _ in range(5):       # duration of the dominant kernel: CUDA events the library records around that launch
@@ -370,8 +420,7 @@ def bench_vector(a, rank, world, out):
 
             def step_b():
                 ix.search_vector_raw(qn, TOPK, hb, nb)
-            msb = timed_steps(step_b, max(10, a.steps), 5, world)
-            per = msb / max(10, a.steps)
+            per = timed_steps(step_b, a.steps, a.warmup, world) / a.steps
             sweep[str(bs)] = {"ms_per_call": per, "queries_per_s": bs / (per / 1e3)}
     best = max(names, key=lambda k: res[k]["value"])      # headline = what SSB_VEC_KERNEL_AUTO picks for this batch size
     r = res[best]
@@ -421,6 +470,7 @@ def bench_vector_int8(a, rank, world):
         ix.search_vector_keys(q_dev, TOPK, keys)
     step_dev(); torch.cuda.synchronize()
     ms = timed_steps(step_dev, a.steps, a.warmup, world)
+    keep_keys("int8", keys, nb)
     kern_ns = []
     for _ in range(5):
         step_dev(); torch.cuda.synchronize()
@@ -440,8 +490,7 @@ def bench_vector_int8(a, rank, world):
 
             def step_b():
                 ix.search_vector_raw(qn, TOPK, hb, nbuf)
-            n_it = max(5, a.steps // 2)
-            per = timed_steps(step_b, n_it, 2, world) / n_it
+            per = timed_steps(step_b, a.steps, a.warmup, world) / a.steps
             sweep[str(bs)] = {"ms_per_call": per, "queries_per_s": bs / (per / 1e3)}
     peak, peak_kind = peaks()
     passes = (nb + 127) // 128
@@ -504,6 +553,7 @@ def bench_vector_int8_variants(a, rank, world):
             ix.search_vector_keys(q_dev, TOPK, keys)
         step_dev(); torch.cuda.synchronize()
         ms = timed_steps(step_dev, a.steps, a.warmup, world)
+        keep_keys(name, keys, nb)
         kern_ns = []
         for _ in range(3):
             step_dev(); torch.cuda.synchronize()
@@ -641,11 +691,11 @@ def bm25_queries(n, seed=2003):
     return [[int(k) for k in synth.term_keys_np(np.array(q, dtype=np.int64))] for q in qs]
 
 
-def _bm25_filter_variants(a, ix, qk, out_keys, steps, world, dev):
+def _bm25_filter_variants(a, ix, qk, out_keys, world, dev):
     """SURVEY 8(f) row 4: the C3 OR queries behind a facet range filter that half of the docs pass (is_facet_filter on every candidate; filtered
     queries are scored and counted doc by doc in lex_generic) — 1024 queries per step, Topk and TopkCount."""
     from seekstorm_b200 import FacetFilter, QueryType, ResultType
-    price = torch.randint(0, 1000, (a.bm25_docs,), dtype=torch.int32).numpy().astype(np.uint32)
+    price = np.random.default_rng(1007).integers(0, 1000, a.bm25_docs, dtype=np.uint32)
     ix.set_facets({"price": price})
     nf = min(1024, len(qk))
     bf, keep_f = ix._lex_batch(qk[:nf], QueryType.Union, None, [[FacetFilter("price", 0, 500)]] * nf)
@@ -654,11 +704,11 @@ def _bm25_filter_variants(a, ix, qk, out_keys, steps, world, dev):
     for name, rt_ in (("or_topk_facet_filter", ResultType.Topk), ("or_topkcount_facet_filter", ResultType.TopkCount)):
         def step_f():
             ix.search_lexical_keys(bf, TOPK, rt_, out_keys, cnt_dev)
-        nv = max(2, steps // 2)
-        msv = timed_steps(step_f, nv, 2, world)
+        msv = timed_steps(step_f, a.steps, a.warmup, world)
+        keep_keys(f"bm25_{name}", out_keys, nf, cnt_dev if rt_ == ResultType.TopkCount else None)
         step_f(); torch.cuda.synchronize()
         sv = ix.last_stats()
-        res[name] = {"value": nf * nv / (msv / 1e3), "unit": "queries/s", "kernel_ms": sv["dominant_kernel_ns"] / 1e6, "queries_per_step": nf,
+        res[name] = {"value": nf * a.steps / (msv / 1e3), "unit": "queries/s", "kernel_ms": sv["dominant_kernel_ns"] / 1e6, "queries_per_step": nf,
                      "selectivity": 0.5, "kernel": "lex_score<.., HAS_NOT> (Topk: filter on the exact-score survivors) / lex_generic (counts: every match tested)"}
     ix.set_facets({})
     return res
@@ -688,14 +738,14 @@ def bench_phrase(a, rank, world):
     cnt_dev = torch.zeros(len(qk), dtype=torch.int64, device=dev)
     res = {"config": {"workload": f"{n} docs Zipf(1) V={C3_VOCAB} with positions ({n_pos} tokens), {len(qk)} phrases/step of 2-3 terms, ranks log-uniform [1,300]",
                       "index_build_s": build_s}}
-    steps = max(3, a.steps // 2)
     for name, rt_ in (("topk", ResultType.Topk), ("topkcount", ResultType.TopkCount)):
         def step():
             ix.search_lexical_keys(b, TOPK, rt_, out_keys, cnt_dev)
-        ms = timed_steps(step, steps, 2, world)
+        ms = timed_steps(step, a.steps, a.warmup, world)
+        keep_keys(f"phrase_{name}", out_keys, len(qk), cnt_dev if rt_ == ResultType.TopkCount else None)
         step(); torch.cuda.synchronize()
         sv = ix.last_stats()
-        res[name] = {"value": len(qk) * steps / (ms / 1e3), "unit": "queries/s", "ms_per_step": ms / steps, "kernel_ms": sv["dominant_kernel_ns"] / 1e6,
+        res[name] = {"value": len(qk) * a.steps / (ms / 1e3), "unit": "queries/s", "ms_per_step": ms / a.steps, "kernel_ms": sv["dominant_kernel_ns"] / 1e6,
                      "postings_visited": sv.get("postings_visited"), "kernel": "lex_generic (intersection + phrase predicate)"}
     res["matching_phrases"] = int((cnt_dev > 0).sum().item())
     ix.close()
@@ -718,8 +768,8 @@ def bench_bm25(a, rank, world, keep_index=False, vector_dims=0):
 
     def step_dev():     # N>1: collective (all-gather + merge of the packed keys inside the library)
         ix.search_lexical_keys(b_dev, TOPK, ResultType.Topk, out_keys)
-    steps = max(3, a.steps // 2)
-    ms = timed_steps(step_dev, steps, a.warmup, world)
+    ms = timed_steps(step_dev, a.steps, a.warmup, world)
+    keep_keys("bm25", out_keys, len(qk))
     kern_ns = []
     for _ in range(3):
         step_dev(); torch.cuda.synchronize()
@@ -731,7 +781,7 @@ def bench_bm25(a, rank, world, keep_index=False, vector_dims=0):
 
     def step_e2e():
         ix.search_lexical_raw(b, TOPK, ResultType.Topk, hits_buf, nh_buf, cnt_buf)   # ssb_search_lexical, host buffers
-    ms_e2e = timed_steps(step_e2e, steps, a.warmup, world)
+    ms_e2e = timed_steps(step_e2e, a.steps, a.warmup, world)
     # secondary modes on the same index / queries (device-resident, same timing rules): exact counts and AND
     variants = {}
     for name, qt_, rt_ in (("or_topkcount", QueryType.Union, ResultType.TopkCount), ("and_topkcount", QueryType.Intersection, ResultType.TopkCount),
@@ -741,28 +791,28 @@ def bench_bm25(a, rank, world, keep_index=False, vector_dims=0):
 
         def step_v():
             ix.search_lexical_keys(bv, TOPK, rt_, out_keys, cnt_dev)
-        nv = max(2, steps // 2)
-        msv = timed_steps(step_v, nv, 2, world)
+        msv = timed_steps(step_v, a.steps, a.warmup, world)
+        keep_keys(f"bm25_{name}", out_keys, len(qk), cnt_dev if rt_ == ResultType.TopkCount else None)
         step_v(); torch.cuda.synchronize()
         sv = ix.last_stats()
-        variants[name] = {"value": len(qk) * nv / (msv / 1e3), "unit": "queries/s", "kernel_ms": sv["dominant_kernel_ns"] / 1e6,
+        variants[name] = {"value": len(qk) * a.steps / (msv / 1e3), "unit": "queries/s", "kernel_ms": sv["dominant_kernel_ns"] / 1e6,
                           "algorithmic_bytes_per_launch": sv["algorithmic_bytes"]}
     if world == 1:
         try:
-            variants.update(_bm25_filter_variants(a, ix, qk, out_keys, steps, world, dev))
+            variants.update(_bm25_filter_variants(a, ix, qk, out_keys, world, dev))
         except Exception as e:  # pragma: no cover
             variants["or_topk_facet_filter"] = {"error": repr(e)}
     peak, peak_kind = peaks()
     kern_ms = float(np.median(kern_ns)) / 1e6 if kern_ns and min(kern_ns) > 0 else None
     alg = st.get("algorithmic_bytes")
     res = {
-        "metric": "queries/sec at top-10 (BM25 OR, block-max pruned, ResultType::Topk)", "value": len(qk) * steps / (ms / 1e3),
-        "unit": "queries/s", "ms_per_step": ms / steps, "steps": steps, "dtype": "f32 scores / u16 postings",
+        "metric": "queries/sec at top-10 (BM25 OR, block-max pruned, ResultType::Topk)", "value": len(qk) * a.steps / (ms / 1e3),
+        "unit": "queries/s", "ms_per_step": ms / a.steps, "steps": a.steps, "dtype": "f32 scores / u16 postings",
         "config": {"workload": f"C3 BM25 OR top-{TOPK}: {a.bm25_docs} docs Zipf(1) V={C3_VOCAB}, {len(qk)} queries/step of 2-4 terms (40/40/20%), ranks log-uniform [20,1e5]",
                    "index_build_s": build_s, "l2": "posting arenas larger than L2 (12 B per posting: stream word, payload, f32 component; %.1f GB per GPU)" % (12 * 0.08 * a.bm25_docs / world / 1e6 / 1e3 * 1e3)},
-        "e2e": {"value": len(qk) * steps / (ms_e2e / 1e3), "unit": "queries/s", "ms_per_step": ms_e2e / steps,
+        "e2e": {"value": len(qk) * a.steps / (ms_e2e / 1e3), "unit": "queries/s", "ms_per_step": ms_e2e / a.steps,
                 "h2d_bytes_per_step": int(keep[0].nbytes + keep[1].nbytes), "d2h_bytes_per_step": len(qk) * (32 * 8 + 8)},
-        "gpu_launches": int(launches) * steps, "variants": variants,
+        "gpu_launches": int(launches) * a.steps, "variants": variants,
         "roofline": {"bound": "hbm", "achieved": (alg / (kern_ms / 1e3) / 1e9) if (alg and kern_ms) else None, "peak": peak, "unit": "GB/s",
                      "frac": (alg / (kern_ms / 1e3) / 1e9 / peak) if (alg and kern_ms) else None,
                      "traffic": NCU["lex_score"]["traffic"] if (a.bm25_docs == C3_DOCS and len(qk) == 4096 and world == 1) else None,
@@ -790,7 +840,7 @@ def _add_vector_levels(ix, n_rows, rank, world, dev, seed_base):
     return local
 
 
-def _hybrid_steps(a, ix, qk, qv, world, steps):
+def _hybrid_steps(a, ix, qk, qv, world, name):
     from seekstorm_b200 import QueryType
     from seekstorm_b200._lib import check, lib
     import ctypes as C
@@ -800,7 +850,8 @@ def _hybrid_steps(a, ix, qk, qv, world, steps):
 
     def step():
         check(lib().ssb_search_hybrid(ix._h, C.byref(b), qv.ctypes.data, TOPK, hits.ctypes.data, nh.ctypes.data))
-    ms = timed_steps(step, steps, 2, world)
+    ms = timed_steps(step, a.steps, a.warmup, world)
+    keep_hits(name, hits, nh)
     launches = ix.last_stats()["kernel_launches"]
     return ms, int(qv.nbytes + keep[0].nbytes + keep[1].nbytes), launches
 
@@ -817,20 +868,19 @@ def bench_hybrid(a, rank, world):
     nq = 1000
     qk = bm25_queries(nq, 2004)
     qv = synth.gen_vectors(nq, C2_DIMS, 2005, "cpu").numpy()
-    steps = max(3, a.steps // 4)
-    ms, h2d, launches = _hybrid_steps(a, ix, qk, qv, world, steps)
+    ms, h2d, launches = _hybrid_steps(a, ix, qk, qv, world, "hybrid")
     ix.close()
     peak, peak_kind = peaks()
     passes = (nq + 255) // 256                                   # AUTO: filter scan, 256 queries per pass over the 2-byte plane
     alg = float(local_rows) * C2_DIMS * 2 * passes
-    return {"metric": "queries/sec at top-10 (hybrid: BM25 OR + 768-d cosine, RRF)", "value": nq * steps / (ms / 1e3), "unit": "queries/s",
-            "ms_per_step": ms / steps, "steps": steps,
+    return {"metric": "queries/sec at top-10 (hybrid: BM25 OR + 768-d cosine, RRF)", "value": nq * a.steps / (ms / 1e3), "unit": "queries/s",
+            "ms_per_step": ms / a.steps, "steps": a.steps,
             "config": {"workload": f"C4 hybrid: {n_docs} docs (Zipf lexical index + {n_docs} x {C2_DIMS} f32 vectors), {nq} queries/step, e2e through ssb_search_hybrid (host buffers)"},
-            "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": nq * 32 * 16, "gpu_launches": int(launches) * steps,
+            "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": nq * 32 * 16, "gpu_launches": int(launches) * a.steps,
             # the step is bounded below by the vector scan: 4 filter passes of 256 queries over the 7.7 GB fp16 plane (f32-equivalent: x2)
-            "roofline": {"bound": "hbm", "achieved": alg / (ms / steps / 1e3) / 1e9, "peak": peak, "unit": "GB/s",
-                         "frac": alg / (ms / steps / 1e3) / 1e9 / peak, "peak_kind": f"of {peak_kind}", "kernel": "whole step (filter scan_tc + refine, lex_score overlapped, host RRF)",
-                         "algorithmic_bytes_per_launch": alg, "f32_equivalent_gbs": 2 * alg / (ms / steps / 1e3) / 1e9}}
+            "roofline": {"bound": "hbm", "achieved": alg / (ms / a.steps / 1e3) / 1e9, "peak": peak, "unit": "GB/s",
+                         "frac": alg / (ms / a.steps / 1e3) / 1e9 / peak, "peak_kind": f"of {peak_kind}", "kernel": "whole step (filter scan_tc + refine, lex_score overlapped, host RRF)",
+                         "algorithmic_bytes_per_launch": alg, "f32_equivalent_gbs": 2 * alg / (ms / a.steps / 1e3) / 1e9}}
 
 
 def bench_c5(a, rank, world, ix):
@@ -846,15 +896,15 @@ def bench_c5(a, rank, world, ix):
     qk = bm25_queries(nq, 2003)
     qv_t = synth.gen_vectors(nq, C2_DIMS, 2006, "cpu").pin_memory()
     qv = qv_t.numpy()
-    steps = max(3, a.steps // 4)
-    ms, h2d, launches = _hybrid_steps(a, ix, qk, qv, world, steps)
+    ms, h2d, launches = _hybrid_steps(a, ix, qk, qv, world, "c5")
     # vector-only on the same shards (device-resident, batch 256): the scan at C5 size
     q_dev = qv_t[:a.batch].to(dev)
     keys = torch.zeros((a.batch, 32), dtype=torch.int64, device=dev)
 
     def step_v():
         ix.search_vector_keys(q_dev, TOPK, keys)
-    msv = timed_steps(step_v, max(3, a.steps // 2), 3, world)
+    msv = timed_steps(step_v, a.steps, a.warmup, world)
+    keep_keys("c5_vector", keys, a.batch)
     kern = []
     for _ in range(3):
         step_v(); torch.cuda.synchronize()
@@ -863,12 +913,12 @@ def bench_c5(a, rank, world, ix):
     passes = (a.batch + 255) // 256 if a.batch > 128 else 1      # AUTO: filter scan (2-byte plane), 256 (128) queries per pass
     alg = float(local_rows) * C2_DIMS * 2 * passes
     kern_ms = float(np.median(kern)) / 1e6 if kern and min(kern) > 0 else None
-    return {"metric": "queries/sec at top-10 (C5: 10M docs BM25 + 10M x 768 cosine, RRF hybrid, sharded)", "value": nq * steps / (ms / 1e3),
-            "unit": "queries/s", "ms_per_step": ms / steps, "steps": steps,
+    return {"metric": "queries/sec at top-10 (C5: 10M docs BM25 + 10M x 768 cosine, RRF hybrid, sharded)", "value": nq * a.steps / (ms / 1e3),
+            "unit": "queries/s", "ms_per_step": ms / a.steps, "steps": a.steps,
             "config": {"workload": f"C5: {n} docs + {n} x {C2_DIMS} f32 vectors over {world} GPU(s) ({local_rows} rows on this rank), {nq} hybrid queries/step, e2e through ssb_search_hybrid",
                        "vector_build_s": build_s},
-            "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": nq * 32 * 16, "gpu_launches": int(launches) * steps,
-            "vector_only": {"value": a.batch * max(3, a.steps // 2) / (msv / 1e3), "unit": "queries/s", "batch": a.batch,
+            "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": nq * 32 * 16, "gpu_launches": int(launches) * a.steps,
+            "vector_only": {"value": a.batch * a.steps / (msv / 1e3), "unit": "queries/s", "batch": a.batch,
                             "roofline": {"bound": "hbm", "achieved": (alg / (kern_ms / 1e3) / 1e9) if kern_ms else None, "peak": peak, "unit": "GB/s",
                                          "frac": (alg / (kern_ms / 1e3) / 1e9 / peak) if kern_ms else None, "peak_kind": f"of {peak_kind}",
                                          "kernel": "scan_tc<256, f16 filter>", "kernel_ms": kern_ms, "algorithmic_bytes_per_launch": alg,
@@ -1000,7 +1050,7 @@ def emit(obj):
 
 
 def main():
-    global _REAL_STDOUT
+    global _REAL_STDOUT, _OUTPUTS
     a = parse()
     # stdout carries exactly one JSON line: everything else any library writes to fd 1 (NCCL prints its version banner
     # there whenever NCCL_DEBUG >= VERSION) is sent to stderr instead
@@ -1037,6 +1087,8 @@ def main():
     if not os.path.exists(g.LIB):
         g.build()
     rank, world = dist_setup(a.gpus)
+    if a.dump_outputs and rank == 0:       # at N>1 every rank returns the merged global results: rank 0 writes them
+        _OUTPUTS = {}
     # one explicit (non-default) stream for everything: library kernels, torch CUDA events and NCCL collectives
     stream = torch.cuda.Stream()
     torch.cuda.set_stream(stream)
@@ -1117,6 +1169,8 @@ def main():
                 out["bm25"]["cpu_baseline"] = cpu_bm25_baseline(a, a.cpu_seconds)
             except Exception as e:  # pragma: no cover
                 out["bm25"]["cpu_baseline"] = {"error": repr(e)}
+    if _OUTPUTS is not None:
+        write_outputs(a.dump_outputs)
     if rank == 0:
         emit(out)
     if world > 1:
